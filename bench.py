@@ -13,6 +13,10 @@ requests at 768x1024 (config 2 of BASELINE.json: batch 2, guidance 2.0), synthet
 
 Launch:  python bench.py [--gpus N --steps K --warmup W]      (N > 1: under torchrun, one rank per GPU, weights
 NCCL-broadcast from rank 0, independent requests per rank — weak scaling, no per-step collective).
+
+--dump-outputs DIR writes the final latents of the last timed step (rank 0's requests, in request order) to
+DIR/latents.npy in float32. Inputs, weights and noise are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -239,6 +243,27 @@ def synth_request(cfg_t, cfg_g, batch, h, w, seed, device, garments=None):
              prompt_embeds=r(2 * batch, 77, cross), add_text_embeds=r(2 * batch, pooled), add_time_ids=tid,
              image_embeds=r(2 * batch, 16, cross), text_embeds_cloth=r(garments, 77, cross))
     return {k: (v.to(device) if k == "add_time_ids" else v.to(device, torch.float16)) for k, v in d.items()}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays, seed=0):
+    """Writes every tensor of `arrays` as <path>/<name>.npy in float32. When they come to more than DUMP_LIMIT_BYTES,
+    each is replaced by a sample of its flattened elements at indices drawn by a generator seeded with `seed`, so the
+    same arguments always select the same elements. Returns the names that were sampled."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    sampled = []
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            idx = np.random.default_rng(seed).choice(a.size, a.size * DUMP_LIMIT_BYTES // total, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+            sampled.append(name)
+        np.save(os.path.join(path, name + ".npy"), a)
+    return sampled
 
 
 # ------------------------------------------------------------------------------------------------
@@ -489,18 +514,24 @@ def run_b200(args, rank, world, local):
             den.step(i, noise, use_graph=True)
         return den.latents
 
-    def run_loop():
+    def run_loop(keep=None):
         """One bench step: the full denoising loop for every batch of this rank (inputs resident in HBM). With one batch
-        per rank the step-invariant context K/V stay prepared; the hoisted garment passes are inside the step."""
+        per rank the step-invariant context K/V stay prepared; the hoisted garment passes are inside the step. `keep`:
+        a list that receives a copy of every batch's final latents (the batches share one latent buffer)."""
         if len(reqs) == 1:
             den.latents.copy_(reqs[0]["latents"])
             if den.hoist_garment:
                 den.precompute_garment(0)    # the garment-UNet passes of this request (batched) + garment K/V
-            return denoise(reqs[0])
+            out = denoise(reqs[0])
+            if keep is not None:
+                keep.append(out.clone())
+            return out
         for req in reqs:
             den.prepare(**req, guidance_scale=GUIDANCE)
             den.set_step_tables(sch, sch.timesteps)        # includes the hoisted garment passes
             out = denoise(req)
+            if keep is not None:
+                keep.append(out.clone())
         return out
 
     den.prepare(**reqs[0], guidance_scale=GUIDANCE)
@@ -521,10 +552,11 @@ def run_b200(args, rank, world, local):
         torch.cuda.profiler.stop()
         log("profiled one denoise step; not a bench run")
         return
+    out = None
     for _ in range(args.warmup):
         out = run_loop()
     torch.cuda.synchronize()
-    assert torch.isfinite(out.float()).all(), "non-finite latents"
+    assert out is None or torch.isfinite(out.float()).all(), "non-finite latents"
     log(f"{args.warmup} warm-up loops done")
 
     def barrier():
@@ -537,10 +569,11 @@ def run_b200(args, rank, world, local):
     evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     barrier()
     eager0 = L.launch_count()
+    last = []                                       # final latents of the last timed step, for --dump-outputs
     with ClockSampler(local) as clocks:
-        for s, e in evs:
+        for k, (s, e) in enumerate(evs):
             s.record()
-            run_loop()
+            run_loop(last if args.dump_outputs and k == len(evs) - 1 else None)
             e.record()
         barrier()
     eager_launches = L.launch_count() - eager0      # launches outside the graph (hoisted garment passes, prepare)
@@ -551,6 +584,9 @@ def run_b200(args, rank, world, local):
         tt = torch.tensor([total_ms], device=device)
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         total_ms = tt.item()
+    if args.dump_outputs and rank == 0:
+        sampled = dump_outputs(args.dump_outputs, {"latents": torch.cat(last)})
+        log(f"outputs of the last timed step written to {args.dump_outputs}" + (f" (sampled: {sampled})" if sampled else ""))
     ms_per_step = total_ms / args.steps
     value = n_requests * args.steps / (total_ms / 1e3)
     log(f"timed region done: {ms_per_step:.1f} ms per bench step, {value:.3f} images/s")
@@ -712,7 +748,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--profile-one-step", action="store_true", help="run one denoise step inside a cudaProfiler range (ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the final latents of the last timed step to DIR/latents.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     # watchdog: a bench that is still running after 20 minutes is stuck (the default run takes ~3 min) — dump every
     # Python stack to stderr and exit non-zero instead of occupying the GPU box until the caller's limit
     import faulthandler

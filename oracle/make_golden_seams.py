@@ -1,14 +1,16 @@
 """Golden vectors for the seam tests (tests/test_seams_gpu.py), produced by the REFERENCE's own code.
 
-Runs only in the build container (needs /root/reference). Imported unmodified and in place:
+Needs a checkout of the original IDM-VTON repository, whose modules are imported unmodified and in place:
   * ip_adapter/attention_processor.py  AttnProcessor2_0 (:189-278), IPAttnProcessor2_0 (:1879-2010), executed on the
     diffusers-shim `Attention` container (oracle/shim/diffusers/models/attention_processor.py), CPU fp32;
   * ip_adapter/resampler.py            Resampler at the geometry the try-on UNet hard-codes
     (src/unet_hacked_tryon.py:476-485: dim 1280, depth 4, 20 heads x 64, 16 queries, CLIP width 1280 -> 2048).
-Writes tests/golden/attn_processors_ref.pt (weights + inputs + outputs, fp16 storage of fp16-representable values so
-every implementation sees identical numbers) and tests/golden/resampler_sdxl_ref.pt (seeds + output).
+Writes tests/golden/attn_processors_ref.pt (self- and cross-attention) and tests/golden/attn_processors_ip_ref.pt
+(IP-Adapter cross-attention): weights + inputs + outputs, fp16 storage of fp16-representable values so every
+implementation sees identical numbers, split in two so that each file stays under 1 MB; and
+tests/golden/resampler_sdxl_ref.pt (seeds + output).
 
-Usage:  python oracle/make_golden_seams.py
+Usage:  python oracle/make_golden_seams.py <path of the IDM-VTON checkout>
 """
 import importlib.util
 import os
@@ -17,7 +19,6 @@ import sys
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
@@ -45,12 +46,12 @@ def resampler_weights(r, seed):
     return sd
 
 
-def main():
+def main(ref):
     sys.path.insert(0, os.path.join(ROOT, "oracle", "shim"))
     sys.path.insert(0, ROOT)
     from diffusers.models.attention_processor import Attention           # the shim's container
-    ap = _load_by_path("ref_attention_processor", os.path.join(REF, "ip_adapter", "attention_processor.py"))
-    rs = _load_by_path("ref_resampler", os.path.join(REF, "ip_adapter", "resampler.py"))
+    ap = _load_by_path("ref_attention_processor", os.path.join(ref, "ip_adapter", "attention_processor.py"))
+    rs = _load_by_path("ref_resampler", os.path.join(ref, "ip_adapter", "resampler.py"))
     os.makedirs(GOLDEN, exist_ok=True)
     g = torch.Generator().manual_seed(2024)
 
@@ -67,7 +68,8 @@ def main():
               "to_out.0.bias": r(C, scale=0.1)}
         a1.load_state_dict(w1, strict=True)
         x = r(B, T, C)
-        out["self"] = dict(weights={k: v.half() for k, v in w1.items()}, x=x.half(), y=a1(x))
+        xh = x.half()                  # one stored copy, shared by every case
+        out["self"] = dict(weights={k: v.half() for k, v in w1.items()}, x=xh, y=a1(x))
         # ---- plain cross-attention (AttnProcessor2_0 with encoder_hidden_states: the garment UNet's attn2)
         a2 = Attention(query_dim=C, cross_attention_dim=cross, heads=heads, dim_head=64, bias=False, out_bias=True,
                        processor=ap.AttnProcessor2_0())
@@ -76,8 +78,8 @@ def main():
               "to_out.0.bias": r(C, scale=0.1)}
         a2.load_state_dict(w2, strict=True)
         enc = r(B, Tt, cross)
-        out["cross"] = dict(weights={k: v.half() for k, v in w2.items()}, x=x.half(), enc=enc.half(),
-                            y=a2(x, encoder_hidden_states=enc))
+        w2h = {k: v.half() for k, v in w2.items()}
+        out["cross"] = dict(weights=w2h, x=xh, enc=enc.half(), y=a2(x, encoder_hidden_states=enc))
         # ---- IP-Adapter decoupled cross-attention (IPAttnProcessor2_0), scale 1.0 (inference) and 0.5
         enc_ip = r(B, Tt + Ti, cross)
         wip = {"to_k_ip.weight": r(C, cross, scale=cross ** -0.5), "to_v_ip.weight": r(C, cross, scale=cross ** -0.5)}
@@ -89,13 +91,17 @@ def main():
                            processor=proc)
             a3.load_state_dict({**w2, **{f"processor.{k}": v for k, v in wip.items()}}, strict=True)
             ys[s] = a3(x, encoder_hidden_states=enc_ip)
-        out["ip"] = dict(weights={k: v.half() for k, v in {**w2, **wip}.items()}, x=x.half(), enc=enc_ip.half(),
-                         y_scale_1=ys[1.0], y_scale_0p5=ys[0.5], num_tokens=Ti)
-    out["note"] = ("outputs (fp32) of the REFERENCE processors ip_adapter/attention_processor.py AttnProcessor2_0 / "
-                   "IPAttnProcessor2_0 on the diffusers-shim Attention container, CPU fp32; weights and inputs are "
-                   "fp16-representable and stored here")
+        ip = dict(weights={**w2h, **{k: v.half() for k, v in wip.items()}}, x=xh, enc=enc_ip.half(),
+                  y_scale_1=ys[1.0], y_scale_0p5=ys[0.5], num_tokens=Ti)
+    note = ("outputs (fp32) of the REFERENCE processors ip_adapter/attention_processor.py AttnProcessor2_0 / "
+            "IPAttnProcessor2_0 on the diffusers-shim Attention container, CPU fp32; weights and inputs are "
+            "fp16-representable and stored here")
+    out["note"] = note + "; the IP-Adapter case is in attn_processors_ip_ref.pt"
     torch.save(out, os.path.join(GOLDEN, "attn_processors_ref.pt"))
-    print("wrote attn_processors_ref.pt", {k: tuple(v["y"].shape) if "y" in v else None for k, v in out.items() if isinstance(v, dict)})
+    torch.save({"C": C, "heads": heads, "ip": ip, "note": note + "; self / cross cases: attn_processors_ref.pt"},
+               os.path.join(GOLDEN, "attn_processors_ip_ref.pt"))
+    print("wrote attn_processors_ref.pt", {k: tuple(v["y"].shape) for k, v in out.items() if isinstance(v, dict)},
+          "and attn_processors_ip_ref.pt", tuple(ip["y_scale_1"].shape))
 
     # ---- Resampler at the SDXL / IDM-VTON geometry, reference module loaded standalone
     rcfg = dict(dim=1280, depth=4, dim_head=64, heads=20, num_queries=16, embedding_dim=1280, output_dim=2048, ff_mult=4)
@@ -120,4 +126,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        raise SystemExit("usage: python oracle/make_golden_seams.py <path of the IDM-VTON checkout>")
+    main(sys.argv[1])

@@ -550,15 +550,8 @@ def _sig(fn):
 
 def test_pipeline_signatures_equal_reference():
     """__init__ / encode_prompt / __call__ / check_inputs: same parameter names, order, defaults and **kwargs as
-    src/tryon_pipeline.py (golden extracted by oracle/make_signature_golden.py; re-extracted live when the reference is
-    present)."""
+    src/tryon_pipeline.py (golden extracted by oracle/make_signature_golden.py)."""
     gold = json.load(open(os.path.join(GOLDEN, "pipeline_signature.json")))["signatures"]
-    ref_path = "/root/reference/src/tryon_pipeline.py"
-    if os.path.exists(ref_path):
-        from oracle.make_signature_golden import extract
-        live = extract(ref_path, "StableDiffusionXLInpaintPipeline", tuple(gold))
-        for k in gold:
-            assert live[k]["args"] == gold[k]["args"] and live[k]["defaults"] == gold[k]["defaults"]
     tree = ast.parse(open(os.path.join(ROOT, "idm-vton_b200", "pipeline.py")).read())
     cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "StableDiffusionXLInpaintPipeline")
     mine = {f.name: _sig(f) for f in cls.body if isinstance(f, ast.FunctionDef) and f.name in gold}

@@ -50,7 +50,7 @@ def test_attn_processors_vs_reference_golden():
     a2 = _attention_from(c["weights"], C, heads, cross, AttnProcessor2_0())
     e_cross = _err(a2(c["x"].cuda(), encoder_hidden_states=c["enc"].cuda()), c["y"])
     # decoupled text + IP cross-attention, scale 1.0 (inference) and 0.5
-    i = g["ip"]
+    i = torch.load(os.path.join(G, "attn_processors_ip_ref.pt"))["ip"]
     errs = []
     for scale, key in ((1.0, "y_scale_1"), (0.5, "y_scale_0p5")):
         proc = IPAttnProcessor2_0(hidden_size=C, cross_attention_dim=cross, scale=scale, num_tokens=i["num_tokens"],
