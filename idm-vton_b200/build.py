@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libb200vton.so")
-SOURCES = ["host.cu", "gemm.cu", "gemm2.cu", "attn.cu", "attn6.cu", "attn_cross.cu", "attn_enc.cu", "conv_tf32.cu", "norm_f32.cu", "vae_f32.cu", "norm.cu", "elementwise.cu", "capi.cu"]
+SOURCES = ["host.cu", "gemm.cu", "gemm2.cu", "attn.cu", "attn6.cu", "attn_cross.cu", "attn_enc.cu", "conv_tf32.cu", "norm_f32.cu", "vae_f32.cu", "norm.cu", "elementwise.cu", "sched.cu", "capi.cu"]
 HEADERS = ["common.cuh", "gemm_common.cuh", "host.h", os.path.join("..", "..", "include", "b200vton.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -52,13 +52,17 @@ void set_attn_qtiles(int n);
 void set_attn_poly(int n);
 int cfg_ddpm_impl(const void* eps, int ldc, int B, int C, int H, int W, const void* latents, const void* noise,
                   const void* coef, int do_cfg, void* out, cudaStream_t stream);
+int cfg_sched_impl(const void* eps, int ldc, int B, int C, int H, int W, const void* latents, const void* noise,
+                   void* hist, const void* coef, int family, int do_cfg, void* out, cudaStream_t stream);
+int nchw_to_nhwc_scaled_impl(const void* src, int Bs, int Cs, int H, int W, const void* scale, void* dst, int Bd,
+                             int ldc, int c_off, cudaStream_t stream);
 }  // namespace vton
 
 #define S(stream) static_cast<cudaStream_t>(stream)
 
 extern "C" {
 
-int b200vton_version(void) { return 106; }
+int b200vton_version(void) { return 107; }
 const char* b200vton_last_error(void) { return vton::get_last_error(); }
 long long b200vton_launch_count(void) { return vton::launch_count(); }
 int b200vton_set_option(const char* name, int value) {
@@ -188,6 +192,15 @@ int b200vton_skinny_linear(const void* x, int ldx, int M, int K, const void* W, 
 int b200vton_cfg_ddpm_step(const void* eps, int ldc, int B, int C, int H, int W, const void* latents,
                            const void* noise, const void* coef, int do_cfg, void* out, void* stream) {
   return vton::cfg_ddpm_impl(eps, ldc, B, C, H, W, latents, noise, coef, do_cfg, out, S(stream));
+}
+int b200vton_cfg_sched_step(const void* eps, int ldc, int B, int C, int H, int W, const void* latents,
+                            const void* noise, void* hist, const void* coef, int family, int do_cfg, void* out,
+                            void* stream) {
+  return vton::cfg_sched_impl(eps, ldc, B, C, H, W, latents, noise, hist, coef, family, do_cfg, out, S(stream));
+}
+int b200vton_nchw_to_nhwc_scaled(const void* src, int Bs, int Cs, int H, int W, const void* scale, void* dst, int Bd,
+                                 int ldc, int c_off, void* stream) {
+  return vton::nchw_to_nhwc_scaled_impl(src, Bs, Cs, H, W, scale, dst, Bd, ldc, c_off, S(stream));
 }
 
 int b200vton_preprocess_inpaint(const void* image, const void* mask, int mask_channels, const void* image_min, int B,

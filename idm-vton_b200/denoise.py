@@ -1,9 +1,11 @@
 """The denoising hot loop of IDM-VTON on the B200 engine (src/tryon_pipeline.py:1765-1866).
 
 Per step the reference runs the garment UNet (batch Bg), zero-pads its 70 features for the CFG-uncond half, runs the
-try-on UNet (batch 2B), applies CFG and the DDPM update. Here one step is a fixed launch sequence over static buffers:
-  latents -> [NCHW->NHWC scatter into the 13(+pad)-channel input] -> garment UNet -> try-on UNet (garment K/V streamed
-  as a second attention segment, uncond half in closed form) -> fused CFG+DDPM
+try-on UNet (batch 2B), applies CFG and the scheduler update. Here one step is a fixed launch sequence over static buffers:
+  latents -> [NCHW->NHWC scatter into the 13(+pad)-channel input, x scale_model_input for Euler] -> garment UNet ->
+  try-on UNet (garment K/V streamed as a second attention segment, uncond half in closed form) -> fused CFG+update
+  (DDPM: b200vton_cfg_ddpm_step; DDIM / Euler / Euler-ancestral / DPM-Solver++: b200vton_cfg_sched_step, fed by the
+  per-step rows of step_plan)
 captured once in a CUDA graph and replayed per step; step-invariant work (cross-attention K/V of text / IP tokens,
 aug_emb, the static input channels) is hoisted to prepare().
 """
@@ -58,6 +60,198 @@ def ddpm_step_coefficients(scheduler, t):
     sigma = var ** 0.5 if t > 0 else torch.tensor(0.0)
     inv_sa = torch.tensor(1.0, dtype=torch.float32) / (a_t ** 0.5)
     return float(b_t ** 0.5), float(inv_sa), float(c0), float(c1), float(sigma)
+
+
+# diffusers scheduler classes by what the engine does with them: the four it runs besides DDPM, and the known ones it
+# refuses (with the reason). Any other class name takes the DDPM path (a caller's own DDPM-family object).
+_SCHED_FAMILIES = {"DDPMScheduler": "ddpm", "DDIMScheduler": "ddim", "EulerDiscreteScheduler": "euler",
+                   "EulerAncestralDiscreteScheduler": "euler_ancestral", "DPMSolverMultistepScheduler": "dpmsolver++"}
+_TWO_EVALS = "second order: two UNet evaluations per step (needs two try-on passes and garment K/V at intermediate timesteps)"
+_SCHED_REFUSED = {
+    "HeunDiscreteScheduler": _TWO_EVALS, "KDPM2DiscreteScheduler": _TWO_EVALS, "KDPM2AncestralDiscreteScheduler": _TWO_EVALS,
+    "DPMSolverSDEScheduler": _TWO_EVALS + " and Brownian-tree noise",
+    "LMSDiscreteScheduler": "linear multistep over up to 4 stored derivatives with integrated coefficients",
+    "PNDMScheduler": "pseudo-numerical multistep with a Runge-Kutta warm-up (several evaluations per timestep)",
+    "UniPCMultistepScheduler": "predictor-corrector: the corrector rewrites the previous update with the new model output",
+    "DEISMultistepScheduler": "multistep update over up to 3 stored predictions not covered by the fused kernel",
+    "DPMSolverSinglestepScheduler": "single-step solver: intermediate UNet evaluations inside each step",
+    "EDMDPMSolverMultistepScheduler": "EDM preconditioning of the model input and output",
+    "EDMEulerScheduler": "EDM preconditioning of the model input and output",
+    "LCMScheduler": "consistency-model boundary conditions", "TCDScheduler": "consistency-model boundary conditions",
+    "IPNDMScheduler": "pseudo-numerical multistep over 4 stored derivatives",
+    "DDIMInverseScheduler": "inversion (the timesteps run upwards)",
+    "CMStochasticIterativeScheduler": "consistency-model sampling",
+}
+
+
+def _cfg_get(scheduler):
+    cfg = getattr(scheduler, "config", None)
+    return (lambda k, d=None: cfg.get(k, d)) if isinstance(cfg, dict) else (lambda k, d=None: getattr(cfg, k, d))
+
+
+def scheduler_family(scheduler):
+    """'ddpm' | 'ddim' | 'euler' | 'euler_ancestral' | 'dpmsolver++' for the caller's scheduler object, named by
+    `config._class_name` when present (what diffusers' from_config records) else by its class name. Unsupported
+    classes and configurations raise NotImplementedError naming the scheduler and the reason; host-only, so a caller
+    can validate before any GPU work."""
+    get = _cfg_get(scheduler)
+    name = get("_class_name", None) or type(scheduler).__name__
+    if name in _SCHED_REFUSED:
+        raise NotImplementedError(f"{name} is not supported by the B200 engine: {_SCHED_REFUSED[name]}")
+    fam = _SCHED_FAMILIES.get(name, "ddpm")
+    if fam == "ddpm":
+        return fam                         # ddpm_step_coefficients checks its own configuration
+    if get("prediction_type", "epsilon") != "epsilon":
+        raise NotImplementedError(f"{name}: prediction_type {get('prediction_type')!r} is not supported (epsilon only)")
+    if get("thresholding", False) or get("clip_sample", False):
+        raise NotImplementedError(f"{name}: thresholding / clip_sample are not supported")
+    if fam == "dpmsolver++":
+        if get("algorithm_type", "dpmsolver++") != "dpmsolver++":
+            raise NotImplementedError(f"{name}: algorithm_type {get('algorithm_type')!r} is not supported (SDE variants "
+                                      "draw noise inside the solver; only 'dpmsolver++' is fused)")
+        if get("solver_order", 2) not in (1, 2):
+            raise NotImplementedError(f"{name}: solver_order {get('solver_order')} is not supported (orders 1 and 2)")
+        if get("use_lu_lambdas", False):
+            raise NotImplementedError(f"{name}: use_lu_lambdas is not supported")
+        if get("solver_type", "midpoint") not in ("midpoint", "heun"):
+            raise NotImplementedError(f"{name}: solver_type {get('solver_type')!r} is not supported")
+        if get("variance_type", None) in ("learned", "learned_range"):
+            raise NotImplementedError(f"{name}: variance_type {get('variance_type')!r} is not supported")
+    return fam
+
+
+class StepPlan:
+    """What the denoise loop needs from the scheduler, per step i: rows[i] (the fused kernel's coefficients after the
+    guidance scale: 5 for DDPM, 7 otherwise, the last being the model-input scale), t[i] (the float timestep fed to the
+    time embedding) and draws[i] (whether the reference's scheduler.step draws noise of the latents' shape)."""
+
+    def __init__(self, family, rows, t, draws):
+        self.family, self.rows, self.t, self.draws = family, rows, t, draws
+
+    @property
+    def scaled_input(self):
+        return self.family in ("euler", "euler_ancestral")
+
+
+def _f32(x):
+    return torch.as_tensor(x, dtype=torch.float32, device="cpu")
+
+
+def step_plan(scheduler, timesteps=None, eta=0.0):
+    """The per-step plan of `scheduler` (after its set_timesteps) over `timesteps` (default: all of scheduler.timesteps; a
+    suffix of them is allowed, as get_timesteps returns). Reads the object's own tables — timesteps, sigmas,
+    alphas_cumprod, config — so spacing variants, Karras sigmas and the final-sigma convention come from it; only the
+    step formulas are restated, in fp32 torch on the CPU like diffusers (see csrc/sched.cu for the row layouts). The
+    scheduler object is not modified and its step() is never called."""
+    fam = scheduler_family(scheduler)
+    all_ts = scheduler.timesteps
+    timesteps = all_ts if timesteps is None else timesteps
+    T, N = len(timesteps), len(all_ts)
+    off = N - T
+    if T == 0 or off < 0 or [float(t) for t in all_ts[off:]] != [float(t) for t in timesteps]:
+        raise ValueError("timesteps must be a suffix of scheduler.timesteps")
+    t_vals = [float(t) for t in timesteps]
+    if fam == "ddpm":
+        rows = [list(ddpm_step_coefficients(scheduler, int(t))) for t in timesteps]
+        return StepPlan(fam, rows, t_vals, [int(t) > 0 for t in timesteps])
+    get = _cfg_get(scheduler)
+    rows = []
+    if fam == "ddim":
+        ac = _f32(scheduler.alphas_cumprod)
+        n_train = int(get("num_train_timesteps", len(ac)))
+        n_inf = getattr(scheduler, "num_inference_steps", None) or N
+        final = getattr(scheduler, "final_alpha_cumprod", None)
+        final = _f32(1.0 if get("set_alpha_to_one", True) else ac[0]) if final is None else _f32(final)
+        for t in timesteps:
+            t = int(t)
+            prev_t = t - n_train // n_inf
+            a_t = ac[t]
+            a_prev = ac[prev_t] if prev_t >= 0 else final
+            b_t, b_prev = 1 - a_t, 1 - a_prev
+            std = eta * ((b_prev / b_t) * (1 - a_t / a_prev)) ** 0.5
+            cdir = (1 - a_prev - std ** 2) ** 0.5
+            rows.append([float(b_t ** 0.5), float(a_t ** 0.5), float(a_prev ** 0.5), float(cdir), float(std), 0.0, 1.0])
+        return StepPlan(fam, rows, t_vals, [eta > 0] * T)
+    sig = _f32(scheduler.sigmas)
+    if fam in ("euler", "euler_ancestral"):
+        for i in range(T):
+            k = off + i
+            s, s_next = sig[k], sig[k + 1]
+            in_scale = _f32(1.0) / ((s ** 2 + 1) ** 0.5)
+            if fam == "euler":
+                sigma_hat = s * (0.0 + 1)
+                rows.append([float(sigma_hat), float(s_next - sigma_hat), 0.0, 0.0, 0.0, 0.0, float(in_scale)])
+            else:
+                up = (s_next ** 2 * (s ** 2 - s_next ** 2) / s ** 2) ** 0.5
+                down = (s_next ** 2 - up ** 2) ** 0.5
+                rows.append([float(s), float(down - s), float(up), 0.0, 0.0, 0.0, float(in_scale)])
+        return StepPlan(fam, rows, t_vals, [True] * T)
+    # DPM-Solver++ (multistep): the solver's own order schedule, replayed from a fresh set_timesteps
+    order = int(get("solver_order", 2))
+    heun = get("solver_type", "midpoint") == "heun"
+
+    def a_s(x):                                         # _sigma_to_alpha_sigma_t
+        alpha = 1 / ((x ** 2 + 1) ** 0.5)
+        return alpha, x * alpha
+
+    def lam(alpha, s):
+        return torch.log(alpha) - torch.log(s)
+
+    for i in range(T):
+        k = off + i
+        lower_final = k == N - 1 and (get("euler_at_final", False) or (get("lower_order_final", True) and N < 15)
+                                      or get("final_sigmas_type", "sigma_min") == "zero")
+        alpha_t, sig_t = a_s(sig[k + 1])
+        alpha_s0, sig_s0 = a_s(sig[k])
+        h = lam(alpha_t, sig_t) - lam(alpha_s0, sig_s0)
+        c1 = alpha_t * (torch.exp(-h) - 1.0)
+        ratio = sig_t / sig_s0
+        c2 = rr = 0.0
+        # a step onto sigma 0 (lambda = +inf, exp(-h) = 0) is taken first order: the second-order term is unbounded there;
+        # so is a zero-length step (h = 0, Karras sigmas ending on sigma_min twice), where its limit is 0
+        if not (order == 1 or i < 1 or lower_final or float(sig[k + 1]) == 0.0 or float(h) == 0.0):
+            alpha_s1, sig_s1 = a_s(sig[k - 1])
+            h_0 = lam(alpha_s0, sig_s0) - lam(alpha_s1, sig_s1)
+            r0 = h_0 / h
+            rr = float(1.0 / r0)
+            c2 = float(alpha_t * ((torch.exp(-h) - 1.0) / h + 1.0)) if heun else -float(0.5 * c1)
+        rows.append([float(sig_s0), float(alpha_s0), float(ratio), float(c1), c2, rr, 1.0])
+    return StepPlan(fam, rows, t_vals, [False] * T)
+
+
+def apply_plan_row(family, row, x, g, noise=None, hist=None):
+    """One step of `family` with plan row `row` in the arithmetic of the input tensors (the fp64 restatement the tests
+    compare with each scheduler's own step(); the engine runs the same formulas in csrc/sched.cu). Divisors are applied
+    as divisions. Returns (prev, x0)."""
+    if family == "ddim":
+        sb, sa, sap, cdir, std = row[:5]
+        x0 = (x - sb * g) / sa
+        prev = sap * x0 + cdir * g
+        if noise is not None and std != 0.0:
+            prev = prev + std * noise
+        return prev, x0
+    if family in ("euler", "euler_ancestral"):
+        sigma, dt = row[0], row[1]
+        x0 = x - sigma * g
+        prev = x + (x - x0) / sigma * dt
+        if family == "euler_ancestral":
+            prev = prev + row[2] * noise
+        return prev, x0
+    if family == "dpmsolver++":
+        sig_s, alpha_s, ratio, c1, c2, rr = row[:6]
+        x0 = (x - sig_s * g) / alpha_s
+        prev = ratio * x - c1 * x0
+        if c2 != 0.0:
+            prev = prev + c2 * (rr * (x0 - hist))
+        return prev, x0
+    raise ValueError(family)
+
+
+def garment_cache_signature(t_values, h, w):
+    """What a cached garment's K/V depend on besides the garment: the timesteps the garment UNet saw (as floats, so
+    Euler's non-integer timesteps get their own entries, while DDPM's keys equal the integer ones: (999.0,) == (999,))
+    and the latent size."""
+    return (tuple(float(t) for t in t_values), h, w)
 
 
 class GarmentKVCache:
@@ -159,7 +353,8 @@ class TryOnDenoiser:
             self.x_t = torch.zeros((Bt, h, w, CIN_PAD), dtype=f16, device=dev)
             self.x_g = torch.zeros((Bg, h, w, CIN_PAD), dtype=f16, device=dev)
             self.t_dev = torch.zeros(1, dtype=torch.float32, device=dev)
-            self.coef = torch.zeros(6, dtype=torch.float32, device=dev)
+            self.coef = torch.zeros(8, dtype=torch.float32, device=dev)     # DDPM reads the first 6
+            self.hist = torch.zeros_like(self.latents)       # DPM-Solver++: the previous step's x0 prediction
             self.step_base = torch.zeros(1, dtype=torch.int32, device=dev)   # step index * Bg (hoisted garment K/V)
             self.ctx_t = self.ctx_g = self.aug = None
             self.eps = None
@@ -172,16 +367,24 @@ class TryOnDenoiser:
         self.ctx_g = self.garment.encode_context(text_embeds_cloth.to(dev, f16), out=self.ctx_g)
         self.aug = self.tryon.aug_embedding(add_text_embeds.to(dev, f16), add_time_ids.to(dev), out=self.aug)
 
-    def set_step_tables(self, scheduler, timesteps, garment_keys=None, cache=None):
-        """Uploads the per-step scalars: t and {gs, sqrt(1-abar), 1/sqrt(abar), c0, c1, sigma}, then runs the hoisted
-        garment passes. garment_keys (one hashable per garment of this batch) + cache (GarmentKVCache): garments whose
-        K/V of all steps are cached are copied in instead of recomputed — valid only when the caller guarantees that a
-        key identifies (cloth latents, text_embeds_cloth); the timestep list and latent size are added to the key here."""
-        rows = []
-        for t in timesteps:
-            rows.append([self.guidance_scale, *ddpm_step_coefficients(scheduler, int(t))])
+    def set_step_tables(self, scheduler, timesteps, garment_keys=None, cache=None, eta=0.0, plan=None):
+        """Uploads the per-step scalars of step_plan(scheduler, timesteps, eta) (or `plan`): t and the fused kernel's
+        coefficient row — DDPM {gs, sqrt(1-abar), 1/sqrt(abar), c0, c1, sigma}, other schedulers see csrc/sched.cu —
+        then runs the hoisted garment passes. A scheduler family other than the one the step graph was captured for
+        drops the graph (recaptured at the next step). garment_keys (one hashable per garment of this batch) + cache
+        (GarmentKVCache): garments whose K/V of all steps are cached are copied in instead of recomputed — valid only
+        when the caller guarantees that a key identifies (cloth latents, text_embeds_cloth); the timestep list and latent
+        size are added to the key here."""
+        plan = plan if plan is not None else step_plan(scheduler, timesteps, eta)
+        if plan.family != getattr(self, "family", None):
+            self._graph = None
+        self.family = plan.family
+        self.plan = plan
+        if plan.family == "dpmsolver++":
+            self.hist.zero_()                            # no x0 prediction of an earlier request leaks in
+        rows = [[self.guidance_scale, *r] for r in plan.rows]
         self.coef_table = torch.tensor(rows, dtype=torch.float32, device=self.device)
-        self.t_table = torch.tensor([float(int(t)) for t in timesteps], dtype=torch.float32, device=self.device)
+        self.t_table = torch.tensor(plan.t, dtype=torch.float32, device=self.device)
         T = len(rows)
         self.window = T
         if self.hoist_garment:
@@ -201,7 +404,7 @@ class TryOnDenoiser:
         if self.hoist_garment:
             use_cache = cache is not None and garment_keys is not None and len(garment_keys) == self.Bg and self.window == T
             if use_cache:
-                sig = (tuple(int(t) for t in timesteps), self.h, self.w)
+                sig = garment_cache_signature(plan.t, self.h, self.w)
                 full = [(k, sig) for k in garment_keys]
                 hit = [cache.get(k) for k in full]
                 if all(e is not None for e in hit):
@@ -277,7 +480,10 @@ class TryOnDenoiser:
     def _launch_step(self):
         """The launch sequence of one denoise step over the static buffers (graph-capturable)."""
         L = self.L
-        L.nchw_to_nhwc(self.latents, self.x_t, c_off=0)          # CFG duplication + channel concat as offsets
+        if self.family in ("euler", "euler_ancestral"):
+            L.nchw_to_nhwc_scaled(self.latents, self.x_t, self.coef[7:8], c_off=0)     # + scale_model_input
+        else:
+            L.nchw_to_nhwc(self.latents, self.x_t, c_off=0)      # CFG duplication + channel concat as offsets
         temb_t = self.tryon.time_embedding(self.t_dev, self.Bt, self.aug)
         n_persons = self.B if self.do_cfg else 0
         if self.gkv_all is not None:
@@ -288,7 +494,11 @@ class TryOnDenoiser:
             temb_g = self.garment.time_embedding(self.t_dev, self.Bg)
             self.garment.forward(self.x_g, temb_g, self.ctx_g, collect=feats)
             self.eps = self.tryon.forward(self.x_t, temb_t, self.ctx_t, gfeats=feats, n_persons=n_persons)
-        L.cfg_ddpm_step(self.eps, self.latents, self.noise, self.coef, do_cfg=self.do_cfg, out=self.latents_next)
+        if self.family == "ddpm":
+            L.cfg_ddpm_step(self.eps, self.latents, self.noise, self.coef, do_cfg=self.do_cfg, out=self.latents_next)
+        else:
+            L.cfg_sched_step(self.eps, self.latents, self.noise, self.hist, self.coef, self.family, do_cfg=self.do_cfg,
+                             out=self.latents_next)
         self.latents.copy_(self.latents_next)
 
     # Programmatic dependent launch INSIDE the captured step only (B200VTON_PDL_GRAPH, default below): every kernel node
@@ -306,6 +516,7 @@ class TryOnDenoiser:
         s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream())
         keep = self.latents.clone()
+        keep_hist = self.hist.clone() if self.family == "dpmsolver++" else None   # the warm-up launch rewrites it
         with torch.cuda.stream(s):
             self._launch_step()
         torch.cuda.current_stream().wait_stream(s)
@@ -321,6 +532,8 @@ class TryOnDenoiser:
             if self.PDL_IN_GRAPH:
                 self.L.set_option("programmatic_launch", pdl_before)
         self.latents.copy_(keep)
+        if keep_hist is not None:
+            self.hist.copy_(keep_hist)
         self._graph = g
 
     def step(self, i, noise=None, use_graph=True):
@@ -328,7 +541,7 @@ class TryOnDenoiser:
         if self.hoist_garment and self.gkv_all is not None and (i // self.window) * self.window != self.win_start:
             self.precompute_garment((i // self.window) * self.window)      # next K/V window (budgeted hoisting)
         self.t_dev.copy_(self.t_table[i:i + 1])
-        self.coef.copy_(self.coef_table[i])
+        self.coef[:self.coef_table.shape[1]].copy_(self.coef_table[i])
         self.step_base.copy_(self.base_table[i:i + 1])
         if noise is not None:
             self.noise.copy_(noise)
@@ -339,7 +552,7 @@ class TryOnDenoiser:
                 if self._graph is None:
                     self.capture()
                     self.t_dev.copy_(self.t_table[i:i + 1])
-                    self.coef.copy_(self.coef_table[i])
+                    self.coef[:self.coef_table.shape[1]].copy_(self.coef_table[i])
                     self.step_base.copy_(self.base_table[i:i + 1])
                 self._graph.replay()
             else:

@@ -39,12 +39,14 @@ SIGNATURES = {
     "b200vton_timestep_embedding": [_vp, _i, _i, _i, _vp, _vp],
     "b200vton_skinny_linear": [_vp, _i, _i, _i, _vp, _i64, _i, _vp, _i, _i, _vp, _i, _vp, _i, _vp],
     "b200vton_cfg_ddpm_step": [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _vp, _vp],
+    "b200vton_cfg_sched_step": [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp],
+    "b200vton_nchw_to_nhwc_scaled": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp],
     "b200vton_preprocess_inpaint": [_vp, _vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp],
     "b200vton_postprocess_image": [_vp, _i, _i, _i, _i, _vp, _vp, _vp],
 }
 
 _lib = None
-ABI_VERSION = 106      # must equal b200vton_version() of the loaded library (bumped with every SIGNATURES change)
+ABI_VERSION = 107      # must equal b200vton_version() of the loaded library (bumped with every SIGNATURES change)
 
 
 def load(build_if_missing=True):
@@ -427,6 +429,18 @@ def nchw_to_nhwc(src, dst, c_off=0):
     return dst
 
 
+def nchw_to_nhwc_scaled(src, dst, scale, c_off=0):
+    """dst[s,y,x,c_off+c] = fp16(src[s % Bs, c, y, x] * scale[0]); scale: fp32 CUDA tensor (one element read)."""
+    lib = load()
+    Bs, Cs, H, W = src.shape
+    assert src.is_contiguous() and dst.is_contiguous()
+    assert scale.dtype == torch.float32 and scale.is_cuda and scale.numel() >= 1
+    rc = lib.b200vton_nchw_to_nhwc_scaled(_p(src), Bs, Cs, H, W, _p(scale), _p(dst), dst.shape[0], dst.shape[-1], c_off,
+                                          _stream())
+    _check(rc, "b200vton_nchw_to_nhwc_scaled")
+    return dst
+
+
 def nhwc_to_nchw(src, C, out=None):
     lib = load()
     B, H, W, ldc = src.shape
@@ -492,6 +506,23 @@ def cfg_ddpm_step(eps, latents, noise, coef, do_cfg=True, out=None):
     rc = lib.b200vton_cfg_ddpm_step(_p(eps), eps.shape[-1], B, C, H, W, _p(latents), _p(noise), _p(coef), int(do_cfg),
                                     _p(out), _stream())
     _check(rc, "b200vton_cfg_ddpm_step")
+    return out
+
+
+SCHED_FAMILIES = {"ddim": 0, "euler": 1, "euler_ancestral": 2, "dpmsolver++": 3}
+
+
+def cfg_sched_step(eps, latents, noise, hist, coef, family, do_cfg=True, out=None):
+    """Fused CFG + scheduler update (csrc/sched.cu). eps: [2B,H,W,ldc] NHWC (or [B,...] without CFG); latents / noise /
+    hist: [B,C,H,W] fp16 (noise / hist may be None where the family does not read them; hist is updated in place);
+    coef: 8 fp32 on device; family: a key of SCHED_FAMILIES."""
+    lib = load()
+    B, C, H, W = latents.shape
+    if out is None:
+        out = torch.empty_like(latents)
+    rc = lib.b200vton_cfg_sched_step(_p(eps), eps.shape[-1], B, C, H, W, _p(latents), _p(noise), _p(hist), _p(coef),
+                                     SCHED_FAMILIES[family], int(do_cfg), _p(out), _stream())
+    _check(rc, "b200vton_cfg_sched_step")
     return out
 
 

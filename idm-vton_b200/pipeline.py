@@ -15,7 +15,7 @@ from typing import Any, Callable, Dict, List, Optional, Tuple, Union
 import torch
 
 from . import clip as _clip
-from .denoise import TryOnDenoiser
+from .denoise import TryOnDenoiser, scheduler_family, step_plan
 from .vae import VaeImageProcessor
 
 PipelineImageInput = Any
@@ -325,7 +325,15 @@ class StableDiffusionXLInpaintPipeline:
         return prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds
 
     def prepare_extra_step_kwargs(self, generator, eta):
-        return {"generator": generator}
+        """src/tryon_pipeline.py: the kwargs `scheduler.step` accepts (DDIM takes `eta`, the others ignore it)."""
+        step = getattr(self.scheduler, "step", None)
+        params = set(inspect.signature(step).parameters.keys()) if step is not None else set()
+        extra = {}
+        if "eta" in params:
+            extra["eta"] = eta
+        if "generator" in params:
+            extra["generator"] = generator
+        return extra
 
     def check_inputs(self, prompt, prompt_2, image, mask_image, height, width, strength, callback_steps, output_type,
                      negative_prompt=None, negative_prompt_2=None, prompt_embeds=None, negative_prompt_embeds=None,
@@ -579,6 +587,7 @@ class StableDiffusionXLInpaintPipeline:
                                       "IDM-VTON inference path (inference.py:397-414)")
         if cloth is None or pose_img is None or text_embeds_cloth is None:
             raise ValueError("cloth, pose_img and text_embeds_cloth are required (src/tryon_pipeline.py:1644-1654,1787)")
+        scheduler_family(self.scheduler)          # an unsupported scheduler raises here, before any GPU work
 
         # 2. call parameters
         if prompt is not None and isinstance(prompt, str):
@@ -604,6 +613,9 @@ class StableDiffusionXLInpaintPipeline:
         if num_inference_steps < 1:
             raise ValueError(f"After adjusting the num_inference_steps by strength parameter: {strength}, the number of pipeline"
                              f"steps is {num_inference_steps} which is < 1 and not appropriate for this pipeline.")
+        # per-step coefficients, timesteps and noise draws of the caller's scheduler (host only; its step() is not called)
+        eta = self.prepare_extra_step_kwargs(generator, eta).get("eta", 0.0)
+        plan = step_plan(self.scheduler, timesteps, eta)
         latent_timestep = timesteps[:1].repeat(batch_size * num_images_per_prompt)
         is_strength_max = strength == 1.0
 
@@ -727,7 +739,7 @@ class StableDiffusionXLInpaintPipeline:
         den.prepare(latents, mask, masked_image_latents, pose_img, cloth, prompt_embeds, add_text_embeds, add_time_ids,
                     image_embeds, text_embeds_cloth.to(device), guidance_scale=self.guidance_scale,
                     do_cfg=self.do_classifier_free_guidance)
-        den.set_step_tables(self.scheduler, timesteps, garment_keys=garment_keys, cache=self.garment_cache)
+        den.set_step_tables(self.scheduler, timesteps, garment_keys=garment_keys, cache=self.garment_cache, plan=plan)
         if trace:
             trace.mark("denoiser.prepare (context K/V, garment passes)")
         with self.progress_bar(total=num_inference_steps) as progress_bar:
@@ -735,7 +747,8 @@ class StableDiffusionXLInpaintPipeline:
                 if self.interrupt:
                     continue
                 step_noise = None
-                if int(t) > 0:                                                               # DDPMScheduler.step
+                if plan.draws[i]:         # the draw the reference's scheduler.step makes (DDPM: t > 0; DDIM: eta > 0;
+                    # Euler / Euler-ancestral: every step), same generator, shape, device and dtype
                     step_noise = randn_tensor(latents.shape, generator=generator, device=device, dtype=latents.dtype)
                 latents = den.step(i, step_noise, use_graph=self.use_cuda_graph)
                 if callback_on_step_end is not None:

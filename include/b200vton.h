@@ -159,6 +159,11 @@ int b200vton_nchw_to_nhwc(const void* src, int Bs, int Cs, int H, int W, void* d
                           void* stream);
 /* dst NCHW [B,C,H,W] = src NHWC [B,H,W,ldc][..., :C] */
 int b200vton_nhwc_to_nchw(const void* src, int B, int C, int H, int W, int ldc, void* dst, void* stream);
+/* b200vton_nchw_to_nhwc with every value multiplied by *scale (one fp32 on the device), rounded once to fp16: the
+ * latent scatter fused with `scheduler.scale_model_input` (sample / sqrt(sigma^2 + 1) of the Euler schedulers,
+ * src/tryon_pipeline.py:1772). */
+int b200vton_nchw_to_nhwc_scaled(const void* src, int Bs, int Cs, int H, int W, const void* scale, void* dst, int Bd,
+                                 int ldc, int c_off, void* stream);
 
 /* nearest-neighbour x2 (diffusers Upsample2D's F.interpolate), NHWC */
 int b200vton_upsample2x_nhwc(const void* src, int B, int H, int W, int C, void* dst, void* stream);
@@ -199,6 +204,17 @@ int b200vton_token_embedding(const void* ids, int rows, int T, int C, int vocab,
  * {guidance_scale, sqrt(1-abar_t), 1/sqrt(abar_t), x0 coeff, x_t coeff, sigma_t}. */
 int b200vton_cfg_ddpm_step(const void* eps, int ldc, int B, int C, int H, int W, const void* latents,
                            const void* noise, const void* coef, int do_cfg, void* out, void* stream);
+
+/* CFG combine + the update of another scheduler (the pipeline's `scheduler.step` at src/tryon_pipeline.py:1823 with
+ * DDIMScheduler, EulerDiscreteScheduler, EulerAncestralDiscreteScheduler or DPMSolverMultistepScheduler in its place).
+ * family: 0 DDIM, 1 Euler, 2 Euler-ancestral, 3 DPM-Solver++ (orders 1 and 2). Layouts as b200vton_cfg_ddpm_step;
+ * coef: 8 fp32 on device {guidance_scale, 6 per-family step scalars, model-input scale} (rounding points and row layout in
+ * csrc/sched.cu). noise: [B,C,H,W] or NULL (required by family 2; DDIM adds it only when its std coefficient is
+ * non-zero; ignored by families 1 and 3). hist: [B,C,H,W] fp16, the previous step's x0 prediction, read and then
+ * overwritten in place (required by family 3, ignored otherwise). */
+int b200vton_cfg_sched_step(const void* eps, int ldc, int B, int C, int H, int W, const void* latents,
+                            const void* noise, void* hist, const void* coef, int family, int do_cfg, void* out,
+                            void* stream);
 
 /* Pre-processing of the inpainting inputs in one launch (diffusers VaeImageProcessor.preprocess for image and mask,
  * the masked image and the latent-resolution mask: src/tryon_pipeline.py:1588-1602, 940-943). image: [B,3,H,W] fp32;
